@@ -11,6 +11,7 @@ finalize [+ all-gather + k-way merge when the index is row-sharded over N GPUs])
     python bench.py --impl reference ...     # the CPU arm: faiss flat search on the host cores (real faiss when importable,
                                              # else the oracle port), plus the reference's own sem_sim_join operator around it
     python bench.py --config c2|c4|c5 ...    # the secondary BASELINE.json configurations, same contract (bench_secondary.py)
+    python bench.py --dump-outputs DIR ...   # also write what the last timed step returned (scores.npy, ids.npy) under DIR
 
 Prints ONE JSON line (rank 0). `value` = device-resident throughput; `e2e` = the plugin's own host-buffer call
 (b2_index_search at N=1: pinned host queries in, host scores + ids out, H2D/D2H inside; at N>1 ShardedIndex.search_host: each
@@ -33,8 +34,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the source tree may be read-only: leave no __pycache__ in it
 
 BLOCK_ROWS = 1 << 16  # data is generated in fixed row blocks so every world size sees the same matrix
+DUMP_BYTES = 64 << 20  # --dump-outputs budget
 
 
 def env_int(name: str, default: int) -> int:
@@ -129,6 +132,24 @@ class ClockSampler:
                     reasons.add(nm)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(power) if power else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir: str, scores, ids) -> None:
+    """Writes what one search of the query batch hands its caller: scores[nq, k] as float32 (scores.npy) and ids[nq, k] as
+    float64 (ids.npy; exact, the ids are below 2**53). Over DUMP_BYTES, a fixed seeded sample of query rows is written instead,
+    in ascending order, with their positions in the batch (rows.npy, float64): the same rows for the same arguments, so two
+    builds can be compared output for output."""
+    import torch
+    nq, k = scores.shape
+    keep = DUMP_BYTES // (k * (4 + 8) + 8)
+    os.makedirs(out_dir, exist_ok=True)
+    if nq > keep:
+        rows = np.sort(np.random.default_rng(0).choice(nq, size=keep, replace=False))
+        sel = torch.from_numpy(rows).to(scores.device)
+        scores, ids = scores[sel], ids[sel]
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "scores.npy"), scores.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "ids.npy"), ids.cpu().numpy().astype(np.float64))
 
 
 def load_peaks() -> tuple[float, str]:
@@ -436,7 +457,13 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-operator", action="store_true", help="skip the DataFrame -> DataFrame leg")
     ap.add_argument("--parity-queries", type=int, default=256)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the scores and ids the last timed step computed as DIR/<name>.npy (headline B200 run only)")
     args, extra = ap.parse_known_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != "c3" or args.impl != "b200"):
+        ap.error("--dump-outputs is supported by the headline B200 run (--config c3 --impl b200)")
     if args.warmup < 3:
         args.warmup = 3
     if args.config != "c3":
@@ -494,9 +521,10 @@ def main() -> None:
         return float(ms.item()) / steps
 
     filt_ms: list[float] = []
+    last_out: list = []  # (scores, ids) of the latest step, for --dump-outputs
 
     def step_dev():
-        index.search(queries, k)
+        last_out[:] = index.search(queries, k)
         filt_ms.append(index.last_filter_ms())
 
     # ---- device-resident throughput --------------------------------------------------------------------------------
@@ -509,6 +537,9 @@ def main() -> None:
         sampler.start()
     ms_step = timed(step_dev, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last_out)
+    last_out.clear()
     st = nv.stats()
     launches_per_step = st["launches"] / max(args.steps, 1) + (1 if world > 1 else 0)  # + the all-gather kernel is NCCL's
     fallback_q = st["fallback_queries"]

@@ -54,27 +54,23 @@ _native_flags = None
 def native_lib():
     """The same source compiled ON THIS HOST with -march=native (AVX-512 where the host has it) and fp contraction, for the TIMED
     CPU arm only (bench.py): the portable liborc.so is built in the build container for x86-64-v3 so that it runs anywhere and
-    keeps -ffp-contract=off for the canonical scorer. Falls back to the portable library when gcc is not available here."""
+    keeps -ffp-contract=off for the canonical scorer. Falls back to the portable library when gcc is not available here.
+    Compiled (about 2 s) into a private temporary directory that is removed once the library is loaded: the source tree may be
+    read-only, and nothing is left behind."""
     global _native_lib, _native_flags
     if _native_lib is not None:
         return _native_lib
     flags = ["-O3", "-march=native", "-mtune=native", "-ffp-contract=fast", "-funroll-loops"]
     try:
-        import hashlib
-        cpu = ""
+        import shutil
+        import tempfile
+        tmp = tempfile.mkdtemp(prefix="liborc_native_")
         try:
-            with open("/proc/cpuinfo") as f:
-                for ln in f:
-                    if ln.startswith("flags"):
-                        cpu = ln
-                        break
-        except OSError:
-            pass
-        tag = hashlib.sha1((cpu + open(_SRC).read()).encode()).hexdigest()[:12]
-        path = os.path.join(_HERE, f"liborc_native_{tag}.so")
-        if not os.path.exists(path):
+            path = os.path.join(tmp, "liborc_native.so")
             subprocess.run(["gcc", *flags, "-fopenmp", "-fPIC", "-shared", "-o", path, _SRC, "-lm"], check=True, capture_output=True, text=True)
-        L = ctypes.CDLL(path)
+            L = ctypes.CDLL(path)
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
         _native_flags = " ".join(flags)
     except Exception:
         L = lib()

@@ -1,17 +1,21 @@
-"""Generates tests/golden/reference_ops.json by running the REFERENCE's own operator code.
+"""Generates tests/golden/reference_ops.json and tests/golden/reference_vs_calls.{json,npz} by running the REFERENCE's own
+operator code.
 
-    PYTHONHASHSEED=0 python tests/golden/make_reference_golden.py        (needs /root/reference; run in the build container)
+    PYTHONHASHSEED=0 python tests/golden/make_reference_golden.py <checkout of lotus-data/lotus>
 
-/root/reference (lotus-data/lotus @ 136ae4f4) is pure Python but cannot be imported as is: litellm, faiss,
+The reference (lotus-data/lotus @ 136ae4f4) is pure Python but cannot be imported as is: litellm, faiss,
 sentence_transformers, backoff, ... are absent from this image. This script
   * satisfies every missing third-party import with an inert mock EXCEPT `faiss`, for which it installs a small stand-in
     module whose IndexFlat / Kmeans / read_index / write_index are backed by the oracle (oracle/faiss_flat.c) and by
     lotus_b200.faiss_io — i.e. the reference's control flow runs unmodified and only faiss's arithmetic is the restatement;
   * runs the reference's real `FaissVS` (lotus/vector_store/faiss_vs.py), `sem_index`, `sem_sim_join`, `sem_search`,
     `sem_dedup`, `sem_cluster_by` (lotus/sem_ops/*.py, lotus/utils.py) on small seeded inputs;
-  * stores inputs and resulting DataFrames as JSON.
+  * stores inputs and resulting DataFrames as JSON;
+  * records every call those operators make on the vector store (index / load_index / get_vectors_from_index / search), with
+    its arguments and FaissVS's answer (reference_vs_calls.*).
 tests/test_reference_golden.py (CPU, oracle-backed test double) and tests/test_gpu_ops.py (B200VS) replay the scenarios
-through lotus_b200's accessors and must reproduce the frames. Nothing reads /root/reference at test time.
+through lotus_b200's accessors and must reproduce the frames; tests/test_gpu_reference_dropin.py replays the recorded calls on
+B200VS and must get FaissVS's answers. Nothing reads the reference at test time.
 """
 import importlib.abc
 import importlib.machinery
@@ -104,7 +108,7 @@ class _Kmeans:
 faiss.index_factory, faiss.write_index, faiss.read_index, faiss.Kmeans = _index_factory, _write_index, _read_index, _Kmeans
 sys.modules["faiss"] = faiss
 sys.meta_path.append(_MockFinder())
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 import lotus  # noqa: E402  (the REFERENCE package)
 from lotus.models import RM  # noqa: E402
 from lotus.vector_store import FaissVS  # noqa: E402
@@ -136,6 +140,50 @@ class RefTableRM(RM):
         return np.stack([np.asarray(self.table[d], dtype=np.float32) for d in docs]).astype(np.float32)
 
 
+class RecordingFaissVS(FaissVS):
+    """The reference's FaissVS, unchanged, with every call the operators make on it written down (arrays kept aside for the
+    .npz; index directories relative to `root`)."""
+
+    def __init__(self, root):
+        super().__init__()
+        self.root, self.calls, self.arrays = root, [], {}
+        self.searching = False  # FaissVS.__call__ reads the subset through get_vectors_from_index: not an operator's call
+
+    def _arr(self, a):
+        name = f"a{len(self.arrays)}"
+        self.arrays[name] = np.asarray(a)
+        return name
+
+    def _dir(self, d):
+        return os.path.relpath(d, self.root)
+
+    def index(self, docs, embeddings, index_dir, **kwargs):
+        super().index(docs, embeddings, index_dir, **kwargs)
+        self.calls.append({"op": "index", "dir": self._dir(index_dir), "docs": [str(v) for v in docs], "embeddings": self._arr(embeddings)})
+
+    def load_index(self, index_dir):
+        super().load_index(index_dir)
+        self.calls.append({"op": "load_index", "dir": self._dir(index_dir)})
+
+    def get_vectors_from_index(self, index_dir, ids):
+        out = super().get_vectors_from_index(index_dir, ids)
+        if self.searching:
+            return out
+        self.calls.append({"op": "get_vectors_from_index", "dir": self._dir(index_dir), "ids": [int(i) for i in ids],
+                           "ids_type": "pandas.Index" if isinstance(ids, pd.Index) else "list", "out": self._arr(out)})
+        return out
+
+    def __call__(self, query_vectors, K, ids=None, **kwargs):
+        self.searching = True
+        try:
+            out = super().__call__(query_vectors, K, ids=ids, **kwargs)
+        finally:
+            self.searching = False
+        self.calls.append({"op": "search", "query": self._arr(query_vectors), "K": int(K), "ids": None if ids is None else [int(i) for i in ids],
+                           "distances": self._arr(out.distances), "indices": self._arr(np.asarray(out.indices, dtype=np.int64))})
+        return out
+
+
 def frame_to_json(df):
     cols = [str(c) for c in df.columns]
     data = []
@@ -149,7 +197,8 @@ def main():
     out = {"_generated_by": "tests/golden/make_reference_golden.py against lotus-data/lotus @ 136ae4f4 (reference code) + oracle-backed faiss stand-in"}
     tmp = tempfile.mkdtemp()
     dim = 32
-    lotus.settings.configure(rm=RefHashRM(dim), vs=FaissVS())
+    vs = RecordingFaissVS(tmp)
+    lotus.settings.configure(rm=RefHashRM(dim), vs=vs)
 
     left = pd.DataFrame({"a": [f"l{i}" for i in range(7)], "v": list(range(7))})
     right = pd.DataFrame({"b": [f"r{i}" for i in range(11)], "v": list(range(11))})
@@ -192,6 +241,10 @@ def main():
     with open(os.path.join(HERE, "reference_ops.json"), "w") as f:
         json.dump(out, f)
     print("wrote tests/golden/reference_ops.json:", {k: (len(v["cases"]) if isinstance(v, dict) and "cases" in v else 1) for k, v in out.items() if not k.startswith("_")})
+    with open(os.path.join(HERE, "reference_vs_calls.json"), "w") as f:
+        json.dump({"_generated_by": out["_generated_by"], "calls": vs.calls}, f)
+    np.savez_compressed(os.path.join(HERE, "reference_vs_calls.npz"), **vs.arrays)
+    print(f"wrote tests/golden/reference_vs_calls.json + .npz: {len(vs.calls)} calls")
 
 
 if __name__ == "__main__":

@@ -88,6 +88,48 @@ def assert_frame_matches_json(df, j):
                 assert a == b, (a, b)
 
 
+def replay_reference_vs_calls(vs, root):
+    """Makes on `vs` every vector-store call the reference's own operators (sem_index, sem_sim_join, sem_search, sem_dedup,
+    sem_cluster_by) made on its FaissVS when tests/golden/reference_ops.json was generated — same arguments, same argument
+    types — and asserts FaissVS's answers (tests/golden/reference_vs_calls.*, make_reference_golden.py). Those operators
+    build their frames from nothing else, so a store that passes answers them as FaissVS did. One documented divergence:
+    past the last candidate (K > rows searched) FaissVS wraps the -1 pad to the last id (faiss_vs.py:71-72); `vs` must
+    pad with -1. Returns the number of calls replayed."""
+    import json
+    import os
+
+    import pandas as pd
+    golden = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    with open(os.path.join(golden, "reference_vs_calls.json")) as f:
+        calls = json.load(f)["calls"]
+    arrays = np.load(os.path.join(golden, "reference_vs_calls.npz"))
+    rows = {}
+    for n, c in enumerate(calls):
+        where = (n, c["op"])
+        if c["op"] == "index":
+            emb = arrays[c["embeddings"]]
+            vs.index(pd.Series(c["docs"]), emb, os.path.join(root, c["dir"]))
+            rows[c["dir"]] = len(emb)
+            assert vs.index_dir == os.path.join(root, c["dir"]), where
+        elif c["op"] == "load_index":
+            vs.load_index(os.path.join(root, c["dir"]))
+            assert vs.index_dir == os.path.join(root, c["dir"]), where
+        elif c["op"] == "get_vectors_from_index":
+            ids = pd.Index(c["ids"]) if c["ids_type"] == "pandas.Index" else c["ids"]
+            got = np.asarray(vs.get_vectors_from_index(os.path.join(root, c["dir"]), ids))
+            assert np.array_equal(bits(got), bits(arrays[c["out"]])), where
+        else:
+            out = vs(arrays[c["query"]], c["K"], ids=c["ids"])
+            D, I = np.asarray(out.distances), np.asarray(out.indices)
+            want_D, want_I = arrays[c["distances"]], arrays[c["indices"]]
+            assert D.shape == want_D.shape and I.shape == want_I.shape, where
+            m = min(c["K"], rows[os.path.relpath(vs.index_dir, root)] if c["ids"] is None else len(c["ids"]))
+            assert np.array_equal(I[:, :m], want_I[:, :m]), where
+            assert np.array_equal(bits(D[:, :m]), bits(want_D[:, :m])), where
+            assert (I[:, m:] == -1).all(), where
+    return len(calls)
+
+
 def _nv():
     from lotus_b200 import _native
     return _native

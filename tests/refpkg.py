@@ -1,13 +1,12 @@
-"""Imports the UNMODIFIED reference package (lotus-data/lotus) for tests and for bench.py's operator-scope reference leg.
+"""Imports the UNMODIFIED reference package (lotus-data/lotus) for bench.py's operator-scope reference leg.
 
-The package lives under baseline/_ref (scripts/install_reference.py; git-ignored, shipped to the GPU box by gpurun) — in the
-build container /root/reference is used when baseline/_ref is absent. Its third-party imports that this image lacks (litellm,
-sentence_transformers, backoff, ...) are satisfied by inert mocks: none of them is on the embedding-similarity path. `faiss` is
+The package lives under baseline/_ref (scripts/install_reference.py; git-ignored). Its third-party imports that this image
+lacks (litellm, sentence_transformers, backoff, ...) are satisfied by inert mocks: none of them is on the embedding-similarity path. `faiss` is
 either the real wheel (if importable), a stand-in handed in by the caller (bench: oracle-backed, to time the reference's
-operator code around it), or an inert mock (drop-in test: B200VS replaces FaissVS, nothing may call faiss).
+operator code around it), or an inert mock (nothing may call faiss).
 
 Importing the reference REGISTERS its accessors and puts `lotus` into sys.modules, which changes what lotus_b200 binds to:
-call this only in a process of its own (the tests run a worker script in a subprocess)."""
+call this only in a process of its own."""
 from __future__ import annotations
 
 import importlib.abc
@@ -40,17 +39,15 @@ class _MockFinder(importlib.abc.MetaPathFinder, importlib.abc.Loader):
 
 
 def reference_dir() -> str | None:
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isfile(os.path.join(cand, "lotus", "__init__.py")):
-            return cand
-    return None
+    cand = os.path.join(ROOT, "baseline", "_ref")
+    return cand if os.path.isfile(os.path.join(cand, "lotus", "__init__.py")) else None
 
 
 def import_reference(faiss_module=None):
     """-> (lotus module, description of what stands for faiss) or (None, reason)."""
     where = reference_dir()
     if where is None:
-        return None, "reference package not found (run scripts/install_reference.py in the build container)"
+        return None, "reference package not found (scripts/install_reference.py puts it under baseline/_ref)"
     mock = list(MISSING)
     faiss_kind = "real faiss wheel"
     if faiss_module is not None:

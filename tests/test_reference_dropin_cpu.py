@@ -1,25 +1,15 @@
-"""CPU dry run of the drop-in worker (tests/ref_dropin_worker.py): the REAL reference package (baseline/_ref, or /root/reference
-in the build container) + lotus_b200.install() + the reference's unmodified operator classes over B200VS, with the native index
-replaced by the oracle-backed fake. Checks the plumbing the GPU test relies on; the numbers come from the oracle here."""
-import json
-import os
-import subprocess
-import sys
-
-import pytest
-
-import refpkg
-
-HERE = os.path.dirname(os.path.abspath(__file__))
+"""CPU dry run of tests/test_gpu_reference_dropin.py: the vector-store calls the reference's own operators made on FaissVS
+(tests/golden/reference_vs_calls.*) are replayed on B200VS with the native index replaced by the oracle-backed fake. Checks
+the host side the GPU test relies on (directory layout, argument types, id remapping, -1 padding); the numbers come from the
+oracle here."""
+from helpers import FakeIndex, replay_reference_vs_calls
 
 
-def test_reference_operators_over_b200vs_plumbing():
-    if refpkg.reference_dir() is None:
-        pytest.skip("reference package not present (scripts/install_reference.py puts it under baseline/_ref)")
-    r = subprocess.run([sys.executable, os.path.join(HERE, "ref_dropin_worker.py")], capture_output=True, text=True, timeout=600,
-                       env=dict(os.environ, B2_TEST_FAKE_NATIVE="1"))
-    assert r.returncode == 0, r.stderr[-3000:]
-    res = json.loads(r.stdout.strip().splitlines()[-1])
-    for name, v in res.items():
-        if isinstance(v, bool):
-            assert v, (name, res)
+def test_reference_vs_calls_replay_over_b200vs_host_logic(monkeypatch, tmp_path):
+    from lotus_b200 import _native as nv
+    from lotus_b200.vs import B200VS
+    monkeypatch.setattr(nv, "Index", FakeIndex)
+    monkeypatch.setattr(nv, "require_device", lambda: None)
+    vs = B200VS(dtype="f32")
+    assert replay_reference_vs_calls(vs, str(tmp_path)) > 0
+    vs.close()
