@@ -55,8 +55,9 @@ extern "C" {
 #define B2_API
 #endif
 
-/* element types of embedding matrices */
-enum { B2_F32 = 0, B2_BF16 = 1 };
+/* element types of embedding matrices (B2_F16: IEEE binary16, the storage of faiss's "SQfp16"). Every entry point that takes
+ * a store dtype or a q_dtype accepts all three, in any combination. */
+enum { B2_F32 = 0, B2_BF16 = 1, B2_F16 = 2 };
 /* metrics; numeric values match faiss.METRIC_INNER_PRODUCT / faiss.METRIC_L2 */
 enum { B2_METRIC_IP = 0, B2_METRIC_L2 = 1 };
 

@@ -11,7 +11,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libb2lotus.so")
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2
 METRIC_IP, METRIC_L2 = 0, 1
 OK, EINVAL, ENODEV, ECUDA, ENOMEM, ERANGE = 0, -1, -2, -3, -4, -5
 
@@ -163,6 +163,29 @@ def bf16_bits_to_f32(b: np.ndarray) -> np.ndarray:
     return out
 
 
+# ---- fp16 helpers (numpy's float16 is IEEE binary16: RNE conversions, so plain numpy does the marshalling) ----------------
+F16_MAX = 65504.0
+
+
+def f32_to_f16_bits(a: np.ndarray) -> np.ndarray:
+    """Round-to-nearest-even float32 -> float16 bit patterns (uint16). Values beyond fp16's range become inf."""
+    with np.errstate(over="ignore"):
+        return np.ascontiguousarray(a, dtype=np.float32).astype(np.float16).view(np.uint16)
+
+
+def f16_bits_to_f32(b: np.ndarray) -> np.ndarray:
+    return np.ascontiguousarray(b, dtype=np.uint16).view(np.float16).astype(np.float32)
+
+
+def bits_to_f32(a: np.ndarray, code: int) -> np.ndarray:
+    """float32 values of a matrix in the library's element type `code` (2-byte types travel as uint16 bit patterns)."""
+    if code == BF16:
+        return bf16_bits_to_f32(a)
+    if code == F16:
+        return f16_bits_to_f32(a)
+    return a
+
+
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else ctypes.c_void_p(a.ctypes.data)
 
@@ -241,6 +264,7 @@ class Index:
                                                       ctypes.c_void_p(stream) if stream else None))
 
     def gather(self, ids) -> np.ndarray:
+        """Rows in the index's element type (uint16 bit patterns for BF16 / F16)."""
         ids = np.ascontiguousarray(ids, dtype=np.int64)
         out = np.empty((len(ids), self.d), dtype=np.float32 if self.dtype == F32 else np.uint16)
         check(lib().b2_index_gather(self._h, _ptr(ids), len(ids), _ptr(out), 0))

@@ -77,13 +77,28 @@ float filter_rel_eps(int store_dtype, int filt_dtype, int q_dtype, int d) {
     const double acc = (double)(d + 64) * 1.1920929e-7;
     double ex = 0.0, eq = 0.0;  // relative representation error of the corpus / query operand seen by the MMA
     if (filt_dtype == B2_F32) {  // kind::tf32 keeps 10 explicit mantissa bits of an fp32 operand
-        ex = store_dtype == B2_F32 ? 9.765625e-4 : 0.0;  // bf16 values are exact in tf32
+        ex = store_dtype == B2_F32 ? 9.765625e-4 : 0.0;  // bf16 and fp16 values (subnormals included) are exact in tf32
         eq = q_dtype == B2_F32 ? 9.765625e-4 : 0.0;
+    } else if (filt_dtype == B2_F16) {  // kind::f16 on fp16 operands: 11 significant bits, exponents 2^-14 .. 2^15
+        // fp32 rounded to fp16: 2^-11 relative in the normal range (the subnormal range is filter_abs_eps's). A bf16 value
+        // (8 significant bits) in the normal range is exact; beyond the finite range prep_queries flags the query.
+        ex = store_dtype == B2_F32 ? 4.8828125e-4 : 0.0;
+        eq = q_dtype == B2_F32 ? 4.8828125e-4 : 0.0;
     } else {  // kind::f16 on bf16 operands
         ex = store_dtype == B2_F32 ? 3.90625e-3 : 0.0;  // fp32 values rounded to bf16 for the filter
-        eq = q_dtype == B2_F32 ? 3.90625e-3 : 0.0;
+        eq = q_dtype != B2_BF16 ? 3.90625e-3 : 0.0;     // fp32 and fp16 queries rounded to bf16 (fp16's range lies inside bf16's)
     }
     return (float)(acc + ex + eq + ex * eq + 1e-6);
+}
+
+// Absolute part of the bound: an operand rounded to fp16 from a type with a wider exponent range (fp32, bf16) may land in
+// fp16's subnormal range, where the rounding error is up to 2^-25 per element whatever the value: 2^-25 sqrt(d) in norm.
+// With ||dq|| <= eq ||q|| + a and ||dx|| <= ex ||x|| + a (a = this value, 0.1 % above 2^-25 sqrt(d) so that the eq a, ex a
+// cross terms are inside it) the inner product moves by at most
+//     rel_eps ||q|| ||x||  +  a (||q|| + ||x|| + a).
+float filter_abs_eps(int store_dtype, int filt_dtype, int q_dtype, int d) {
+    if (filt_dtype != B2_F16 || (store_dtype == B2_F16 && q_dtype == B2_F16)) return 0.f;
+    return (float)(1.001 * 2.98023223876953125e-8 * sqrt((double)d));
 }
 
 // deferred[j] = base + sel[j] (chunk-local query numbers -> batch-wide)
@@ -185,14 +200,21 @@ int search_core(b2_index* idx, const MatView& X_in, int metric, const void* q_de
         int32_t* sel_count = idx->sel.as<int32_t>();
         int32_t* sel_list = sel_count + 1;
         B2_CUDA(cudaMemsetAsync(sel_count, 0, sizeof(int32_t), st));
-        if (!q_in_place) B2_TRY(launch_prep_queries(qc, q_dtype, nqc, X.d, idx->q_filt.p, filt_dtype, q_pitch, st));
+        // fp16 filter operands: queries with an element beyond fp16's finite range are flagged here and answered exactly
+        int32_t* q_bad = nullptr;
+        if (!q_in_place && filt_dtype == B2_F16) {
+            B2_TRY(idx->q_bad.ensure((size_t)nqc * sizeof(int32_t)));
+            q_bad = idx->q_bad.as<int32_t>();
+            B2_CUDA(cudaMemsetAsync(q_bad, 0, (size_t)nqc * sizeof(int32_t), st));
+        }
+        if (!q_in_place) B2_TRY(launch_prep_queries(qc, q_dtype, nqc, X.d, idx->q_filt.p, filt_dtype, q_pitch, st, q_bad));
         B2_CUDA(cudaEventRecord(idx->ev0, st));
         B2_TRY(launch_knn_filter(X, q_filt, q_pitch, nqc, metric, kp, n_splits, two_cta, idx->cand_score.as<float>(),
                                  idx->cand_id.as<int32_t>(), idx->cand_thr.as<float>(), idx->device, st, false, units_whole));
         B2_CUDA(cudaEventRecord(idx->ev1, st));
         B2_TRY(launch_finalize(X, qc, q_dtype, nqc, metric, k, kp, kp / 2, 2 * n_splits, idx->cand_score.as<float>(),
                                idx->cand_id.as<int32_t>(), idx->cand_thr.as<float>(), rel_eps, id_map, id_offset, osc, oid,
-                               idx->flags.as<int32_t>(), sel_list, sel_count, st));
+                               idx->flags.as<int32_t>(), sel_list, sel_count, st, nullptr, q_bad));
         // the certificate outcome comes back as ONE counter (the failed queries are compacted on the device)
         int32_t* h_count = reinterpret_cast<int32_t*>(idx->h_flags.p);
         B2_CUDA(cudaMemcpyAsync(h_count, sel_count, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -291,7 +313,7 @@ int b2_index_create(const void* x, int64_t n, int32_t d, int32_t dtype, int32_t 
     if (!out) { set_error("out is NULL"); return B2_EINVAL; }
     *out = nullptr;
     if (n < 0 || d <= 0 || (n > 0 && !x)) { set_error("bad matrix shape n=%lld d=%d", (long long)n, d); return B2_EINVAL; }
-    if (dtype != B2_F32 && dtype != B2_BF16) { set_error("dtype must be B2_F32 or B2_BF16"); return B2_EINVAL; }
+    if (dtype != B2_F32 && dtype != B2_BF16 && dtype != B2_F16) { set_error("dtype must be B2_F32, B2_BF16 or B2_F16"); return B2_EINVAL; }
     if (metric != B2_METRIC_IP && metric != B2_METRIC_L2) { set_error("metric must be B2_METRIC_IP or B2_METRIC_L2"); return B2_EINVAL; }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
@@ -339,7 +361,7 @@ int b2_index_create(const void* x, int64_t n, int32_t d, int32_t dtype, int32_t 
 void b2_index_free(b2_index* idx) {
     if (!idx) return;
     DeviceGuard guard(idx->device);
-    DevBuf* bufs[] = {&idx->store, &idx->filt_pad, &idx->filt16, &idx->sub_filt16, &idx->defer, &idx->q_sub, &idx->sub_sc, &idx->sub_id, &idx->q_norm2, &idx->norm2, &idx->scalar, &idx->q_in, &idx->q_filt, &idx->cand_score,
+    DevBuf* bufs[] = {&idx->store, &idx->filt_pad, &idx->filt16, &idx->sub_filt16, &idx->defer, &idx->q_sub, &idx->sub_sc, &idx->sub_id, &idx->q_norm2, &idx->q_bad, &idx->norm2, &idx->scalar, &idx->q_in, &idx->q_filt, &idx->cand_score,
                       &idx->cand_id, &idx->cand_thr, &idx->flags, &idx->sel, &idx->dense, &idx->out_sc, &idx->out_id,
                       &idx->ids_dev, &idx->sub_store, &idx->sub_filt, &idx->sub_norm2, &idx->sort_keys};
     for (DevBuf* b : bufs) b->release();
@@ -363,7 +385,7 @@ float b2_last_filter_ms(const b2_index* idx) { return idx ? idx->last_filter_ms 
 static int check_search_args(b2_index* idx, const void* q, int64_t nq, int32_t q_dtype, int32_t k) {
     if (!idx) { set_error("Index not loaded"); return B2_EINVAL; }
     if (nq < 0 || (nq > 0 && !q)) { set_error("bad query batch"); return B2_EINVAL; }
-    if (q_dtype != B2_F32 && q_dtype != B2_BF16) { set_error("q_dtype must be B2_F32 or B2_BF16"); return B2_EINVAL; }
+    if (q_dtype != B2_F32 && q_dtype != B2_BF16 && q_dtype != B2_F16) { set_error("q_dtype must be B2_F32, B2_BF16 or B2_F16"); return B2_EINVAL; }
     if (k <= 0) { set_error("k must be positive (got %d)", k); return B2_EINVAL; }
     if (k > dense_max_k()) { set_error("k=%d is not supported (max %d)", k, dense_max_k()); return B2_ERANGE; }
     return B2_OK;
@@ -493,9 +515,15 @@ int b2_index_search_stage1_dev(b2_index* idx, const void* q_dev, int64_t nq, int
     const int filt_dtype = X.filt_dtype;
     const int64_t q_pitch = round_up(X.d, filt_dtype == B2_F32 ? 4 : 8);
     const bool q_in_place = q_dtype == filt_dtype && q_pitch == X.d && (reinterpret_cast<uintptr_t>(q_dev) & 15) == 0;
+    sg.q_bad = !q_in_place && filt_dtype == B2_F16;
+    if (sg.q_bad) {
+        B2_TRY(idx->q_bad.ensure((size_t)nq * sizeof(int32_t)));
+        B2_CUDA(cudaMemsetAsync(idx->q_bad.p, 0, (size_t)nq * sizeof(int32_t), st));
+    }
     if (!q_in_place) {
         B2_TRY(idx->q_filt.ensure((size_t)nq * q_pitch * esize(filt_dtype)));
-        B2_TRY(launch_prep_queries(q_dev, q_dtype, nq, X.d, idx->q_filt.p, filt_dtype, q_pitch, st));
+        B2_TRY(launch_prep_queries(q_dev, q_dtype, nq, X.d, idx->q_filt.p, filt_dtype, q_pitch, st,
+                                   sg.q_bad ? idx->q_bad.as<int32_t>() : nullptr));
     }
     const void* q_filt = q_in_place ? q_dev : idx->q_filt.p;
     B2_TRY(idx->cand_score.ensure((size_t)nq * n_splits * kp * sizeof(float)));
@@ -510,10 +538,12 @@ int b2_index_search_stage1_dev(b2_index* idx, const void* q_dev, int64_t nq, int
     sg.kp = kp;
     sg.n_splits = n_splits;
     sg.rel_eps = filter_rel_eps(X.dtype, filt_dtype, q_dtype, X.d);
+    sg.abs_eps = filter_abs_eps(X.dtype, filt_dtype, q_dtype, X.d);
     sg.filtered = true;
     B2_TRY(launch_row_norms(q_dev, q_dtype, nq, X.d, idx->q_norm2.as<float>(), idx->scalar.as<float>() + 8, st));
     B2_TRY(launch_shard_lower_bound(idx->cand_score.as<float>(), idx->cand_id.as<int32_t>(), nq, 2 * n_splits, kp / 2, j, idx->q_norm2.as<float>(),
-                                    X.max_norm, sg.rel_eps, idx->metric, lower_dev, st));
+                                    X.max_norm, sg.rel_eps, sg.abs_eps, sg.q_bad ? idx->q_bad.as<int32_t>() : nullptr, idx->metric,
+                                    lower_dev, st));
     g_stats[ST_QUERIES] += nq;
     return B2_OK;
 }
@@ -541,7 +571,8 @@ int b2_index_search_stage2_packed_dev(b2_index* idx, const float* hint_dev, uint
     B2_CUDA(cudaMemsetAsync(sel_count, 0, sizeof(int32_t), st));
     B2_TRY(launch_finalize(X, sg.q, sg.q_dtype, nq, idx->metric, k, sg.kp, sg.kp / 2, 2 * sg.n_splits, idx->cand_score.as<float>(),
                            idx->cand_id.as<int32_t>(), idx->cand_thr.as<float>(), sg.rel_eps, nullptr, 0, idx->out_sc.as<float>(),
-                           idx->out_id.as<int64_t>(), idx->flags.as<int32_t>(), sel_list, sel_count, st, hint_dev));
+                           idx->out_id.as<int64_t>(), idx->flags.as<int32_t>(), sel_list, sel_count, st, hint_dev,
+                           sg.q_bad ? idx->q_bad.as<int32_t>() : nullptr));
     int32_t* h_count = reinterpret_cast<int32_t*>(idx->h_flags.p);
     B2_CUDA(cudaMemcpyAsync(h_count, sel_count, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     cudaError_t se = cudaStreamSynchronize(st);

@@ -16,9 +16,18 @@ __device__ __forceinline__ double butterfly_sum(double v) {
     return v;
 }
 
+// exact float32 value of element i of a B2_F32 / B2_BF16 / B2_F16 array (both 2-byte types widen exactly)
 __device__ __forceinline__ float elem_f32(const void* base, int dtype, size_t i) {
-    return dtype == B2_F32 ? reinterpret_cast<const float*>(base)[i]
-                           : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(base)[i]);
+    if (dtype == B2_F32) return reinterpret_cast<const float*>(base)[i];
+    if (dtype == B2_F16) return __half2float(reinterpret_cast<const __half*>(base)[i]);
+    return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(base)[i]);
+}
+
+// the four fp16 values packed in two 32-bit words, widened
+__device__ __forceinline__ void f16x4_to_f32(uint2 t, float (&o)[4]) {
+    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&t.x));
+    const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&t.y));
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
 }
 
 // 4 consecutive elements of group g of a row (zero beyond d). `vec` = row start is 4-element aligned.
@@ -28,6 +37,8 @@ __device__ __forceinline__ void load_group(const void* row, int dtype, int g, in
         if (dtype == B2_F32) {
             const float4 t = __ldg(reinterpret_cast<const float4*>(row) + g);
             o[0] = t.x; o[1] = t.y; o[2] = t.z; o[3] = t.w;
+        } else if (dtype == B2_F16) {
+            f16x4_to_f32(__ldg(reinterpret_cast<const uint2*>(row) + g), o);
         } else {
             const uint2 t = __ldg(reinterpret_cast<const uint2*>(row) + g);
             o[0] = __uint_as_float(t.x << 16);

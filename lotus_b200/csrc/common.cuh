@@ -1,6 +1,7 @@
 // common.cuh — shared declarations for libb2lotus.so (sm_100a only).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <cfloat>
@@ -78,8 +79,8 @@ __host__ __device__ __forceinline__ float best_first_unkey(uint32_t k, int metri
 }
 
 // ---- a matrix the kernels can search ---------------------------------------------------------------------
-// `store` holds the exact values (dtype f32 or bf16, row pitch `d`). `filt` is what the tcgen05 filter
-// streams through TMA: bf16 (pitch multiple of 8 elements) for a bf16 index, fp32 (pitch multiple of 4)
+// `store` holds the exact values (dtype f32, bf16 or f16, row pitch `d`). `filt` is what the tcgen05 filter
+// streams through TMA: bf16 / fp16 (pitch multiple of 8 elements) for a bf16 / fp16 index, fp32 (pitch multiple of 4)
 // read as TF32 for an fp32 index; it aliases `store` whenever the pitch already qualifies.
 struct MatView {
     const void* store = nullptr;
@@ -88,7 +89,7 @@ struct MatView {
     int64_t n = 0;
     int32_t d = 0;
     int32_t dtype = B2_F32;       // element type of `store`
-    int32_t filt_dtype = B2_F32;  // element type of `filt`: B2_BF16 -> kind::f16 MMA, B2_F32 -> kind::tf32 MMA
+    int32_t filt_dtype = B2_F32;  // element type of `filt`: B2_BF16 / B2_F16 -> kind::f16 MMA, B2_F32 -> kind::tf32 MMA
     int64_t filt_pitch = 0;  // elements
     // fp32 stores only (optional): a bf16 rounding of the rows, pitch multiple of 8. When present, searches run a FIRST level on it
     // (kind::f16 at twice the tf32 rate, operand error 2^-8 per fp32 operand in the certificate) and only the queries whose
@@ -101,6 +102,15 @@ struct MatView {
 };
 
 struct SearchWorkspace;
+
+// ---- certificate margins (api.cu) -----------------------------------------------------------------------------
+// |filter inner product - exact inner product| <= rel ||q|| ||x|| + abs (||q|| + ||x|| + abs), rel = filter_rel_eps(...),
+// abs = filter_abs_eps(...) (non-zero only when an fp32 / bf16 operand is rounded to fp16, whose subnormals lose bits)
+float filter_rel_eps(int store_dtype, int filt_dtype, int q_dtype, int d);
+float filter_abs_eps(int store_dtype, int filt_dtype, int q_dtype, int d);
+__host__ __device__ __forceinline__ double filter_ip_err(double rel, double abs_eps, double qn, double xn) {
+    return rel * qn * xn + abs_eps * (qn + xn + abs_eps);
+}
 
 // ---- kernels / launchers (one per .cu) ------------------------------------------------------------------
 // knn_filter_sm100.cu
@@ -116,12 +126,15 @@ int launch_pair_filter(const MatView& X, float thr, int part, int nparts, int32_
                        unsigned long long* pair_count, unsigned long long cap, int device, cudaStream_t stream);
 
 // knn_exact.cu
+// bad (nullable, [nq], zeroed by the caller): set to 1 for a query with an element that is not a finite filter operand (beyond
+// fp16's range when filt_dtype == B2_F16); its filter row is written with a zero there and finalize sends it to the exact path
 int launch_prep_queries(const void* q, int q_dtype, int64_t nq, int d, void* q_filt, int filt_dtype,
-                        int64_t filt_pitch, cudaStream_t stream);
+                        int64_t filt_pitch, cudaStream_t stream, int32_t* bad = nullptr);
 int launch_row_norms(const void* x, int dtype, int64_t n, int d, float* norm2, float* max_norm_dev,
                      cudaStream_t stream);
+// bad (nullable): set to 1 when an fp16 output element is not finite (it is written as 0)
 int launch_convert_pad(const void* x, int dtype, int64_t n, int d, void* out, int out_dtype, int64_t out_pitch,
-                       cudaStream_t stream);
+                       cudaStream_t stream, int32_t* bad = nullptr);
 int launch_exact_l2_assigned(const void* pts, int dtype, int64_t m, int d, const float* cent, const int64_t* assign, float* out,
                              cudaStream_t stream);
 int launch_gather_rows(const void* x, int dtype, int d, const int64_t* ids, int64_t m, int64_t n, void* out,
@@ -129,10 +142,12 @@ int launch_gather_rows(const void* x, int dtype, int d, const int64_t* ids, int6
 int launch_finalize(const MatView& X, const void* q, int q_dtype, int64_t nq, int metric, int k, int kp, int list_len,
                     int n_lists, const float* cand_score, const int32_t* cand_id, const float* cand_thr,
                     float rel_eps, const int64_t* id_map, int64_t id_offset, float* out_scores, int64_t* out_idx,
-                    int32_t* flags, int32_t* sel, int32_t* sel_count, cudaStream_t stream, const float* hint = nullptr);
+                    int32_t* flags, int32_t* sel, int32_t* sel_count, cudaStream_t stream, const float* hint = nullptr,
+                    const int32_t* q_bad = nullptr);
 int shard_lower_bound_max_entries();
 int launch_shard_lower_bound(const float* cand_score, const int32_t* cand_id, int64_t nq, int n_lists, int list_len, int j, const float* qnorm2,
-                             float max_norm, float rel_eps, int metric, float* lower, cudaStream_t stream);
+                             float max_norm, float rel_eps, float abs_eps, const int32_t* q_bad, int metric, float* lower,
+                             cudaStream_t stream);
 int launch_fill_f32(float* p, int64_t n, float v, cudaStream_t stream);
 int launch_dense_topk(const MatView& X, const void* q, int q_dtype, int64_t nq, const int32_t* q_sel,
                       int64_t n_sel, int metric, int k, const int64_t* id_map, int64_t id_offset, float* dense_ws,

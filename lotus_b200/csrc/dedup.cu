@@ -20,6 +20,11 @@ __device__ __forceinline__ void load_group2(const char* row, int dtype, int g, i
         if (dtype == B2_F32) {
             const float4 t = __ldg(reinterpret_cast<const float4*>(row) + g);
             o[0] = t.x; o[1] = t.y; o[2] = t.z; o[3] = t.w;
+        } else if (dtype == B2_F16) {
+            const uint2 t = __ldg(reinterpret_cast<const uint2*>(row) + g);
+            const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&t.x));
+            const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&t.y));
+            o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
         } else {
             const uint2 t = __ldg(reinterpret_cast<const uint2*>(row) + g);
             o[0] = __uint_as_float(t.x << 16);
@@ -31,9 +36,10 @@ __device__ __forceinline__ void load_group2(const char* row, int dtype, int g, i
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
             const int i = i0 + e;
-            o[e] = i < d ? (dtype == B2_F32 ? reinterpret_cast<const float*>(row)[i]
-                                            : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(row)[i]))
-                         : 0.f;
+            o[e] = i >= d             ? 0.f
+                   : dtype == B2_F32 ? reinterpret_cast<const float*>(row)[i]
+                   : dtype == B2_F16 ? __half2float(reinterpret_cast<const __half*>(row)[i])
+                                     : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(row)[i]);
         }
     }
 }

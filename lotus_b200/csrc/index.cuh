@@ -101,14 +101,15 @@ struct b2_index {
         const void* q = nullptr;
         int64_t nq = 0;
         int32_t q_dtype = 0, k = 0, kp = 0, n_splits = 0;
-        float rel_eps = 0.f;
+        float rel_eps = 0.f, abs_eps = 0.f;
+        bool q_bad = false;  // idx->q_bad holds the queries prep_queries flagged (fp16 filter operands)
     } staged;
-    DevBuf q_norm2;
+    DevBuf q_norm2, q_bad;
 };
 
 namespace b2 {
 
-static inline size_t esize(int dtype) { return dtype == B2_F32 ? 4 : 2; }
+static inline size_t esize(int dtype) { return dtype == B2_F32 ? 4 : 2; }  // B2_BF16, B2_F16: 2 bytes
 
 // searchable view (filter operand, row norms, max norm) of a row-major device matrix
 int build_view(const void* store, int64_t n, int d, int dtype, DevBuf& filt_pad, DevBuf& norm2, DevBuf& scalar, MatView& v,

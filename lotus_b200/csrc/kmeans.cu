@@ -79,8 +79,7 @@ __global__ void rows_to_f32_kernel(const void* x, int dtype, int d, const int64_
         const int64_t r = t / d;
         const int c = (int)(t - r * d);
         const int64_t src = ids ? ids[r] : r;
-        out[t] = dtype == B2_F32 ? reinterpret_cast<const float*>(x)[src * d + c]
-                                 : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(x)[src * d + c]);
+        out[t] = elem_f32(x, dtype, (size_t)(src * d + c));
     }
 }
 
@@ -88,7 +87,7 @@ __global__ void rows_to_f32_kernel(const void* x, int dtype, int d, const int64_
 // cand_* hold, per point and per list (2 epilogue sets x n_splits), the best two (score, centroid) pairs in slots 0-1 and the
 // third-best score in cand_thr (-inf when the list saw fewer than three centroids). score = 2 x.c - ||c||^2 (larger = nearer).
 __global__ void km_assign_finalize_kernel(const float* cand_score, const int32_t* cand_id, const float* cand_thr, int64_t m, int n_lists,
-                                          int list_len, const float* pnorm2, const float* max_norm_dev, float rel_eps, int64_t* assign,
+                                          int list_len, const float* pnorm2, const float* max_norm_dev, float rel_eps, float abs_eps, int64_t* assign,
                                           int32_t* flag_local, int32_t* flag_count, int64_t base) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= m) return;
@@ -114,7 +113,7 @@ __global__ void km_assign_finalize_kernel(const float* cand_score, const int32_t
     const double qn2 = (double)pnorm2[base + i];
     const double qn = sqrt(qn2);
     // |filter score - exact score| for any centroid (same bound as finalize_kernel's L2 certificate)
-    const double eps_s = 2.0 * (double)rel_eps * qn * mx + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1e-30;
+    const double eps_s = 2.0 * filter_ip_err((double)rel_eps, (double)abs_eps, qn, mx) + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1e-30;
     // the reported distances are fp32 roundings of ||x||^2 - score: two exact scores further apart than this cannot round equal
     const double slack = 2.4e-7 * (qn2 + fmax(fabs((double)f1), fabs((double)f2)));
     const bool certain = c1 >= 0 && ((double)f1 - (double)f2) > 2.0 * eps_s + slack;  // false for NaN scores as well
@@ -129,7 +128,7 @@ __global__ void km_assign_finalize_kernel(const float* cand_score, const int32_t
 // reach the exact winner. Points that fail it go on to the general pipeline (hard_ids).
 __global__ void km_rescore_known_kernel(const void* pts, int dtype, int d, const float* cent, const float* cand_score, const int32_t* cand_id,
                                         const float* cand_thr, int n_lists, int list_len, const float* pnorm2, const float* max_norm_dev,
-                                        float rel_eps, const int32_t* flag_local, const int32_t* flag_count, int64_t base, int64_t* assign,
+                                        float rel_eps, float abs_eps, const int32_t* flag_local, const int32_t* flag_count, int64_t base, int64_t* assign,
                                         int64_t* hard_ids, int32_t* hard_count) {
     extern __shared__ __align__(16) float rk_q[];  // [warps per block][d4]
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -159,7 +158,7 @@ __global__ void km_rescore_known_kernel(const void* pts, int dtype, int d, const
         }
         const double qn2 = (double)pnorm2[gi];
         const double qn = sqrt(qn2);
-        const double eps_s = 2.0 * (double)rel_eps * qn * mx + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1.3e-7 * qn2 + 1e-30;
+        const double eps_s = 2.0 * filter_ip_err((double)rel_eps, (double)abs_eps, qn, mx) + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1.3e-7 * qn2 + 1e-30;
         const double slack = 2.4e-7 * (qn2 + fabs((double)f1));
         const bool contender = id >= 0 && (double)f >= (double)f1 - 2.0 * eps_s - slack;
         // recorded candidates that are not contenders count as discarded rows: fold them into the bound
@@ -356,17 +355,17 @@ template <> struct LaneWord<4> { using T = uint32_t; };
 // LB = bytes of a member row per lane (4, 8 or 16): a warp covers 32 * LB contiguous bytes of every member row. Small LB = more,
 // shorter-per-row chains: the time of the pass is bounded below by (largest cluster) x (cycles per row of ONE warp), and the
 // largest cluster is ~10x the mean while Lloyd converges on the benchmark mixture (48k of 5M rows at k = 1024).
-template <bool BF16, bool OBJ, int LB, int ACC_GROUPS>
+template <int DT, bool OBJ, int LB, int ACC_GROUPS>  // DT: element type of the rows (B2_F32, B2_BF16 or B2_F16)
 __global__ void __launch_bounds__(256) km_accumulate_vec_kernel(const void* x, int d, const int64_t* ids, const int32_t* members,
                                                                 const int64_t* offsets, const int32_t* order, const float* cent_old,
                                                                 float* cent_out, float* hassign, double* obj, int normalize, int k,
                                                                 int n_chunks, int* work_counter, long long* dbg) {
-    constexpr int V = BF16 ? LB / 2 : LB / 4;  // columns per lane
+    constexpr int V = DT != B2_F32 ? LB / 2 : LB / 4;  // columns per lane
     using Word = typename LaneWord<LB>::T;
     extern __shared__ __align__(16) uint8_t acc_ring_raw[];  // [warps][ACC_GROUPS * ACC_ROWS][32] words
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     Word* my_ring = reinterpret_cast<Word*>(acc_ring_raw) + (size_t)wib * (ACC_GROUPS * ACC_ROWS * 32) + lane;
-    const size_t row_bytes = (size_t)d * (BF16 ? 2 : 4);
+    const size_t row_bytes = (size_t)d * (DT != B2_F32 ? 2 : 4);
     const int row_words = (int)(row_bytes / LB);
     const int n_items = k * n_chunks;
     for (;;) {
@@ -416,7 +415,14 @@ __global__ void __launch_bounds__(256) km_accumulate_vec_kernel(const void* x, i
         auto consume_row = [&](const Word& raw) {
             float v[V];
             const uint32_t* w32 = reinterpret_cast<const uint32_t*>(&raw);
-            if constexpr (BF16) {
+            if constexpr (DT == B2_F16) {
+#pragma unroll
+                for (int t = 0; t < LB / 4; ++t) {
+                    const float2 h = __half22float2(*reinterpret_cast<const __half2*>(&w32[t]));
+                    v[2 * t] = h.x;
+                    v[2 * t + 1] = h.y;
+                }
+            } else if constexpr (DT == B2_BF16) {
 #pragma unroll
                 for (int t = 0; t < LB / 4; ++t) {
                     v[2 * t] = __uint_as_float(w32[t] << 16);
@@ -517,8 +523,7 @@ __global__ void km_accumulate_kernel(const void* x, int dtype, int d, const int6
         for (int64_t o = o0; o < o1; ++o) {
             const int64_t p = members[o];
             const int64_t r = ids ? ids[p] : p;
-            const float v = dtype == B2_F32 ? reinterpret_cast<const float*>(x)[r * d + j]
-                                            : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(x)[r * d + j]);
+            const float v = elem_f32(x, dtype, (size_t)(r * d + j));
             acc = __fadd_rn(acc, v);
             if (cent_old) {
                 const float df = v - cold;
@@ -631,18 +636,22 @@ __global__ void __launch_bounds__(256) km_split_kernel(int d, int k, int64_t n, 
     }
 }
 
-// searchable view of the fp32 centroid matrix; the filter operand matches the point dtype (bf16 points -> bf16 copy).
+// searchable view of the fp32 centroid matrix; the filter operand matches the point dtype (bf16 / fp16 points -> a bf16 / fp16
+// copy; the fp16 rounding of the centroids is in the certificate through filter_rel_eps / filter_abs_eps).
 // No host synchronisation: the max norm stays in device memory (MatView::max_norm_dev).
 int centroid_view(const float* cent, int k, int d, int point_dtype, KmWork& w, MatView& v, cudaStream_t st) {
     v.store = cent;
     v.n = k;
     v.d = d;
     v.dtype = B2_F32;
-    if (point_dtype == B2_BF16) {
-        v.filt_dtype = B2_BF16;
+    if (point_dtype == B2_BF16 || point_dtype == B2_F16) {
+        v.filt_dtype = point_dtype;
         v.filt_pitch = round_up(d, 8);
         B2_TRY(w.cent_filt.ensure((size_t)k * v.filt_pitch * 2));
-        B2_TRY(launch_convert_pad(cent, B2_F32, k, d, w.cent_filt.p, B2_BF16, v.filt_pitch, st));
+        B2_TRY(w.scalar.ensure(64));
+        int32_t* overflow = reinterpret_cast<int32_t*>(w.scalar.as<char>() + 32);  // read back by assign_points
+        B2_CUDA(cudaMemsetAsync(overflow, 0, sizeof(int32_t), st));
+        B2_TRY(launch_convert_pad(cent, B2_F32, k, d, w.cent_filt.p, point_dtype, v.filt_pitch, st, overflow));
         v.filt = w.cent_filt.p;
     } else {
         v.filt_dtype = B2_F32;
@@ -681,6 +690,7 @@ int assign_points(b2_index* idx, const void* pts, const float* pnorm2, int64_t m
     const int kp = 16;
     const int64_t q_pitch = round_up(d, filt_dtype == B2_F32 ? 4 : 8);
     const float rel_eps = filter_rel_eps(B2_F32, filt_dtype, idx->dtype, d);
+    const float abs_eps = filter_abs_eps(B2_F32, filt_dtype, idx->dtype, d);
     const bool q_in_place = idx->dtype == filt_dtype && q_pitch == d && (reinterpret_cast<uintptr_t>(pts) & 15) == 0;
     const int64_t chunk = (int64_t)1 << 23;
     B2_TRY(w.flag_ids.ensure((size_t)std::min(m, chunk) * sizeof(int32_t)));
@@ -717,13 +727,13 @@ int assign_points(b2_index* idx, const void* pts, const float* pnorm2, int64_t m
         if (q0 > 0) B2_CUDA(cudaMemsetAsync(flag_count, 0, sizeof(int32_t), st));
         km_assign_finalize_kernel<<<(unsigned)ceil_div(mc, 256), 256, 0, st>>>(
             idx->cand_score.as<float>(), idx->cand_id.as<int32_t>(), idx->cand_thr.as<float>(), mc, 2 * n_splits, kp / 2, pnorm2,
-            cv.max_norm_dev, rel_eps, assign, w.flag_ids.as<int32_t>(), flag_count, q0);
+            cv.max_norm_dev, rel_eps, abs_eps, assign, w.flag_ids.as<int32_t>(), flag_count, q0);
         B2_LAUNCH_CHECK();
         // the flagged points of this chunk, while its candidate lists are still in the workspace (count read on the device)
         if (4 * n_splits <= 32)
             km_rescore_known_kernel<<<dev_sms * 4, 256, rk_smem, st>>>(pts, idx->dtype, d, cent, idx->cand_score.as<float>(),
                                                                      idx->cand_id.as<int32_t>(), idx->cand_thr.as<float>(), 2 * n_splits, kp / 2,
-                                                                     pnorm2, cv.max_norm_dev, rel_eps, w.flag_ids.as<int32_t>(), flag_count, q0,
+                                                                     pnorm2, cv.max_norm_dev, rel_eps, abs_eps, w.flag_ids.as<int32_t>(), flag_count, q0,
                                                                      assign, w.hard_ids.as<int64_t>(), hard_count);
         else
             km_forward_flags_kernel<<<dev_sms, 256, 0, st>>>(w.flag_ids.as<int32_t>(), flag_count, q0, w.hard_ids.as<int64_t>(), hard_count);
@@ -731,10 +741,16 @@ int assign_points(b2_index* idx, const void* pts, const float* pnorm2, int64_t m
     }
     int32_t* h_count = reinterpret_cast<int32_t*>(w.h_count.p);
     B2_CUDA(cudaMemcpyAsync(h_count, hard_count, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    h_count[1] = 0;
+    if (filt_dtype == B2_F16) B2_CUDA(cudaMemcpyAsync(h_count + 1, w.scalar.as<char>() + 32, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     cudaError_t se = cudaStreamSynchronize(st);
     if (se != cudaSuccess) {
         set_error("k-means assignment failed on the device: %s", cudaGetErrorString(se));
         return B2_ECUDA;
+    }
+    if (h_count[1]) {  // the fp16 filter copy of a centroid would not be finite: no certificate can hold
+        set_error("a k-means centroid has an element beyond the fp16 range (|x| >= 65520) of this fp16 store");
+        return B2_ERANGE;
     }
     float ms = -1.f;
     if (cudaEventElapsedTime(&ms, idx->ev0, idx->ev1) == cudaSuccess) idx->last_filter_ms = ms;
@@ -837,11 +853,14 @@ int update_centroids(b2_index* idx, const void* x, const int64_t* row_ids, int64
         else B2_ACC_LAUNCH(BF, OB, 4, 32);             \
     } while (0)
         if (idx->dtype == B2_BF16) {
-            if (want_obj) B2_ACC_LB(true, true);
-            else B2_ACC_LB(true, false);
+            if (want_obj) B2_ACC_LB(B2_BF16, true);
+            else B2_ACC_LB(B2_BF16, false);
+        } else if (idx->dtype == B2_F16) {
+            if (want_obj) B2_ACC_LB(B2_F16, true);
+            else B2_ACC_LB(B2_F16, false);
         } else {
-            if (want_obj) B2_ACC_LB(false, true);
-            else B2_ACC_LB(false, false);
+            if (want_obj) B2_ACC_LB(B2_F32, true);
+            else B2_ACC_LB(B2_F32, false);
         }
 #undef B2_ACC_LB
 #undef B2_ACC_LAUNCH

@@ -119,14 +119,30 @@ __device__ __forceinline__ uint64_t warp_merge_keep_low(uint64_t (&buf)[R], cons
 }
 
 // ---- small utility kernels -------------------------------------------------------------------------------------
-__global__ void prep_queries_kernel(const void* q, int q_dtype, int64_t nq, int d, void* out, int out_dtype, int64_t pitch) {
+// one element of a filter operand in out_dtype (round to nearest even); false when the result is not finite
+__device__ __forceinline__ bool store_operand(void* out, int out_dtype, int64_t t, float v) {
+    if (out_dtype == B2_F32) {
+        reinterpret_cast<float*>(out)[t] = v;
+        return true;
+    }
+    if (out_dtype == B2_F16) {
+        __half h = __float2half_rn(v);
+        const bool fin = !__hisinf(h) && !__hisnan(h);
+        reinterpret_cast<__half*>(out)[t] = fin ? h : __float2half_rn(0.f);
+        return fin;
+    }
+    reinterpret_cast<__nv_bfloat16*>(out)[t] = __float2bfloat16_rn(v);
+    return true;
+}
+
+__global__ void prep_queries_kernel(const void* q, int q_dtype, int64_t nq, int d, void* out, int out_dtype, int64_t pitch,
+                                    int32_t* bad) {
     const int64_t total = nq * pitch;
     for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = t / pitch;
         const int c = (int)(t - r * pitch);
         const float v = c < d ? elem_f32(q, q_dtype, (size_t)(r * d + c)) : 0.f;
-        if (out_dtype == B2_F32) reinterpret_cast<float*>(out)[t] = v;
-        else reinterpret_cast<__nv_bfloat16*>(out)[t] = __float2bfloat16_rn(v);
+        if (!store_operand(out, out_dtype, t, v) && bad) bad[r] = 1;
     }
 }
 
@@ -154,14 +170,13 @@ __global__ void row_norms_kernel(const void* x, int dtype, int64_t n, int d, flo
     if (lane == 0 && local_max > 0.f) atomicMax(reinterpret_cast<int*>(max_norm), __float_as_int(local_max));
 }
 
-__global__ void convert_pad_kernel(const void* x, int dtype, int64_t n, int d, void* out, int out_dtype, int64_t pitch) {
+__global__ void convert_pad_kernel(const void* x, int dtype, int64_t n, int d, void* out, int out_dtype, int64_t pitch, int32_t* bad) {
     const int64_t total = n * pitch;
     for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = t / pitch;
         const int c = (int)(t - r * pitch);
         const float v = c < d ? elem_f32(x, dtype, (size_t)(r * d + c)) : 0.f;
-        if (out_dtype == B2_F32) reinterpret_cast<float*>(out)[t] = v;
-        else reinterpret_cast<__nv_bfloat16*>(out)[t] = __float2bfloat16_rn(v);
+        if (!store_operand(out, out_dtype, t, v) && bad) *bad = 1;
     }
 }
 
@@ -193,7 +208,7 @@ __global__ void gather_rows_kernel(const char* x, size_t row_bytes, const int64_
 
 // Canonical partials of U rows at once (vectorisable rows only): the U independent row loads of a step are issued
 // back to back, so each lane keeps U gathers in flight. Per row the accumulation order is exactly canonical_partial's.
-template <bool IS_L2, bool BF16, int U>
+template <bool IS_L2, int DT, int U>  // DT: element type of the rows (B2_F32, B2_BF16 or B2_F16)
 __device__ __forceinline__ void canonical_partial_multi(const float* q_s, const char* const (&rows)[U], int d, int lane,
                                                         double (&acc)[U]) {
 #pragma unroll
@@ -201,7 +216,13 @@ __device__ __forceinline__ void canonical_partial_multi(const float* q_s, const 
     const int ngroups = d >> 2;
     for (int g = lane; g < ngroups; g += 32) {
         float x[U][4];
-        if constexpr (BF16) {
+        if constexpr (DT == B2_F16) {
+            uint2 t[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) t[u] = __ldg(reinterpret_cast<const uint2*>(rows[u]) + g);
+#pragma unroll
+            for (int u = 0; u < U; ++u) f16x4_to_f32(t[u], x[u]);
+        } else if constexpr (DT == B2_BF16) {
             uint2 t[U];
 #pragma unroll
             for (int u = 0; u < U; ++u) t[u] = __ldg(reinterpret_cast<const uint2*>(rows[u]) + g);
@@ -255,8 +276,9 @@ struct FinalizeParams {
     int64_t id_offset;
     int32_t d, dtype, q_dtype, metric, k, kp, n_splits;  // n_splits = number of candidate lists per query, kp = survivors kept
     int32_t list_len;                                    // entries per candidate list (<= 32*R)
-    float rel_eps, max_norm;
+    float rel_eps, abs_eps, max_norm;  // filter error: filter_ip_err(rel_eps, abs_eps, ||q||, ||x||)
     const float* max_norm_dev;  // nullable: overrides max_norm
+    const int32_t* q_bad;       // nullable: queries whose filter operand is not finite (prep_queries): never certified
     const float* hint;          // nullable: per query, a lower bound (filter-score space) on the k-th exact score of the WHOLE
                                 // row-sharded search (b2_index_search_stage1_dev + all-reduce MIN over the ranks)
 };
@@ -339,8 +361,8 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_kernel(const Finalize
     }
     // margin between a filter score and the exact score it stands for (same quantity the certificate uses below)
     const double qn_m = sqrt(qn2), mx_m = (double)max_norm;
-    const double eps_f = is_l2 ? 2.0 * (double)p.rel_eps * qn_m * mx_m + 2.4e-7 * (mx_m * mx_m + 2.0 * qn_m * mx_m) + 1e-30
-                               : (double)p.rel_eps * qn_m * mx_m + 1e-30;
+    const double ip_err = filter_ip_err((double)p.rel_eps, (double)p.abs_eps, qn_m, mx_m);
+    const double eps_f = is_l2 ? 2.0 * ip_err + 2.4e-7 * (mx_m * mx_m + 2.0 * qn_m * mx_m) + 1e-30 : ip_err + 1e-30;
     // Pruning before the (expensive) re-score: the k best survivors BY FILTER SCORE have exact scores >= t_k - eps, so a
     // survivor whose filter score is below t_k - 2 eps is strictly worse than k others: it cannot enter or tie the top k.
 #pragma unroll
@@ -385,11 +407,14 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_kernel(const Finalize
             for (int u = 0; u < 4; ++u)
                 rows[u] = reinterpret_cast<const char*>(p.store) + (size_t)(ids[u] >= 0 ? ids[u] : ids[0]) * p.d * esz;
             if (p.dtype == B2_BF16) {
-                if (is_l2) canonical_partial_multi<true, true, 4>(q_s, rows, p.d, lane, part);
-                else canonical_partial_multi<false, true, 4>(q_s, rows, p.d, lane, part);
+                if (is_l2) canonical_partial_multi<true, B2_BF16, 4>(q_s, rows, p.d, lane, part);
+                else canonical_partial_multi<false, B2_BF16, 4>(q_s, rows, p.d, lane, part);
+            } else if (p.dtype == B2_F16) {
+                if (is_l2) canonical_partial_multi<true, B2_F16, 4>(q_s, rows, p.d, lane, part);
+                else canonical_partial_multi<false, B2_F16, 4>(q_s, rows, p.d, lane, part);
             } else {
-                if (is_l2) canonical_partial_multi<true, false, 4>(q_s, rows, p.d, lane, part);
-                else canonical_partial_multi<false, false, 4>(q_s, rows, p.d, lane, part);
+                if (is_l2) canonical_partial_multi<true, B2_F32, 4>(q_s, rows, p.d, lane, part);
+                else canonical_partial_multi<false, B2_F32, 4>(q_s, rows, p.d, lane, part);
             }
         } else {
 #pragma unroll
@@ -474,21 +499,22 @@ __global__ void __launch_bounds__(FIN_WARPS * 32) finalize_kernel(const Finalize
     const int tie_src0 = (is_l2 || nvalid <= k) ? c : c + m - t;
 
     // 6. certification against everything the filter discarded
-    bool certified = true;
+    // a query the filter could not see as finite operands has meaningless filter scores: the exact path answers it
+    bool certified = !(p.q_bad && p.q_bad[q]);
     // everything the filter discarded scores (exactly) at most bound + eps: below the sharded search's k-th score -> irrelevant
     const bool hint_ok = hint > -INFINITY && ((double)bound + eps_f) < hint - hint_slack;
-    if (bound > -INFINITY && !hint_ok) {
+    if (certified && bound > -INFINITY && !hint_ok) {
         if (nvalid < k) {
             certified = false;  // cannot happen (lists only overflow when full); be safe
         } else {
             const double qn = sqrt(qn2);
             const double v = (double)best_first_unkey((uint32_t)(s_keys[k - 1] >> 32), p.metric);
             if (!is_l2) {
-                const double eps = (double)p.rel_eps * qn * (double)max_norm + 1e-30;
+                const double eps = filter_ip_err((double)p.rel_eps, (double)p.abs_eps, qn, (double)max_norm) + 1e-30;
                 certified = ((double)bound + eps) < v;
             } else {
                 const double mx = (double)max_norm;
-                const double eps_s = 2.0 * (double)p.rel_eps * qn * mx + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1e-30;
+                const double eps_s = 2.0 * filter_ip_err((double)p.rel_eps, (double)p.abs_eps, qn, mx) + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1e-30;
                 // discarded rows have exact L2 >= qn2 - (bound + eps_s); allow for the fp32 rounding of v
                 certified = (qn2 - (double)bound - eps_s) > v * (1.0 + 2.4e-7) + 1e-30;
             }
@@ -825,10 +851,15 @@ __global__ void exact_l2_assigned_kernel(const void* pts, int dtype, int64_t m, 
 // the index are known to score at least that much. Warp per query; up to 32 * LB_R candidate entries.
 constexpr int LB_R = 32;
 __global__ void shard_lower_bound_kernel(const float* cand_score, const int32_t* cand_id, int64_t nq, int n_lists, int list_len, int j,
-                                         const float* qnorm2, float max_norm, float rel_eps, int metric, float* lower) {
+                                         const float* qnorm2, float max_norm, float rel_eps, float abs_eps, const int32_t* q_bad,
+                                         int metric, float* lower) {
     const int lane = threadIdx.x & 31;
     const int64_t q = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     if (q >= nq) return;
+    if (q_bad && q_bad[q]) {  // no finite filter operand: no bound
+        if (lane == 0) lower[q] = -INFINITY;
+        return;
+    }
     const int total = n_lists * list_len;
     float v[LB_R];
 #pragma unroll
@@ -866,8 +897,9 @@ __global__ void shard_lower_bound_kernel(const float* cand_score, const int32_t*
         float out = -INFINITY;
         if (tj > -INFINITY) {
             const double qn = sqrt((double)qnorm2[q]), mx = (double)max_norm;
-            const double eps = metric == B2_METRIC_L2 ? 2.0 * (double)rel_eps * qn * mx + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1.3e-7 * qn * qn + 1e-30
-                                                      : (double)rel_eps * qn * mx * (1.0 + 1.3e-7) + 1e-30;
+            const double ip_err = filter_ip_err((double)rel_eps, (double)abs_eps, qn, mx);
+            const double eps = metric == B2_METRIC_L2 ? 2.0 * ip_err + 2.4e-7 * (mx * mx + 2.0 * qn * mx) + 1.3e-7 * qn * qn + 1e-30
+                                                      : ip_err * (1.0 + 1.3e-7) + 1e-30;
             out = (float)((double)tj - eps - 4.8e-7 * fabs((double)tj));
         }
         lower[q] = out;
@@ -890,9 +922,9 @@ int dense_max_k() { return 1 << 24; }
 int dense_select_max_k() { return SEL_MAX_K; }
 
 int launch_prep_queries(const void* q, int q_dtype, int64_t nq, int d, void* q_filt, int filt_dtype,
-                        int64_t filt_pitch, cudaStream_t stream) {
+                        int64_t filt_pitch, cudaStream_t stream, int32_t* bad) {
     if (nq <= 0) return B2_OK;
-    prep_queries_kernel<<<grid_for(nq * filt_pitch, 256), 256, 0, stream>>>(q, q_dtype, nq, d, q_filt, filt_dtype, filt_pitch);
+    prep_queries_kernel<<<grid_for(nq * filt_pitch, 256), 256, 0, stream>>>(q, q_dtype, nq, d, q_filt, filt_dtype, filt_pitch, bad);
     B2_LAUNCH_CHECK();
     return B2_OK;
 }
@@ -908,10 +940,11 @@ int launch_row_norms(const void* x, int dtype, int64_t n, int d, float* norm2, f
 int shard_lower_bound_max_entries() { return 32 * LB_R; }
 
 int launch_shard_lower_bound(const float* cand_score, const int32_t* cand_id, int64_t nq, int n_lists, int list_len, int j, const float* qnorm2,
-                             float max_norm, float rel_eps, int metric, float* lower, cudaStream_t stream) {
+                             float max_norm, float rel_eps, float abs_eps, const int32_t* q_bad, int metric, float* lower,
+                             cudaStream_t stream) {
     if (nq <= 0) return B2_OK;
     shard_lower_bound_kernel<<<(unsigned)ceil_div(nq * 32, 128), 128, 0, stream>>>(cand_score, cand_id, nq, n_lists, list_len, j, qnorm2, max_norm,
-                                                                                  rel_eps, metric, lower);
+                                                                                  rel_eps, abs_eps, q_bad, metric, lower);
     B2_LAUNCH_CHECK();
     return B2_OK;
 }
@@ -939,9 +972,9 @@ int launch_exact_l2_assigned(const void* pts, int dtype, int64_t m, int d, const
 }
 
 int launch_convert_pad(const void* x, int dtype, int64_t n, int d, void* out, int out_dtype, int64_t out_pitch,
-                       cudaStream_t stream) {
+                       cudaStream_t stream, int32_t* bad) {
     if (n <= 0) return B2_OK;
-    convert_pad_kernel<<<grid_for(n * out_pitch, 256), 256, 0, stream>>>(x, dtype, n, d, out, out_dtype, out_pitch);
+    convert_pad_kernel<<<grid_for(n * out_pitch, 256), 256, 0, stream>>>(x, dtype, n, d, out, out_dtype, out_pitch, bad);
     B2_LAUNCH_CHECK();
     return B2_OK;
 }
@@ -976,10 +1009,13 @@ static int launch_finalize_r(const FinalizeParams& p, cudaStream_t stream) {
 int launch_finalize(const MatView& X, const void* q, int q_dtype, int64_t nq, int metric, int k, int kp, int list_len,
                     int n_splits, const float* cand_score, const int32_t* cand_id, const float* cand_thr,
                     float rel_eps, const int64_t* id_map, int64_t id_offset, float* out_scores, int64_t* out_idx,
-                    int32_t* flags, int32_t* sel, int32_t* sel_count, cudaStream_t stream, const float* hint) {
+                    int32_t* flags, int32_t* sel, int32_t* sel_count, cudaStream_t stream, const float* hint,
+                    const int32_t* q_bad) {
     if (nq <= 0) return B2_OK;
     FinalizeParams p;
     p.hint = hint;
+    p.q_bad = q_bad;
+    p.abs_eps = filter_abs_eps(X.dtype, X.filt_dtype, q_dtype, X.d);
     p.sel = sel;
     p.sel_count = sel_count;
     p.store = X.store;
@@ -1055,7 +1091,7 @@ int launch_dense_topk(const MatView& X, const void* q, int q_dtype, int64_t nq, 
         const int sc = (int)std::min<int64_t>(dense_ws_rows, n_sel - s0);
         const int32_t* sel = q_sel ? q_sel + s0 : nullptr;
         // without a selection list the batch is the contiguous query range [s0, s0+sc)
-        const void* qb = q_sel ? q : reinterpret_cast<const char*>(q) + (size_t)s0 * X.d * (q_dtype == B2_F32 ? 4 : 2);
+        const void* qb = q_sel ? q : reinterpret_cast<const char*>(q) + (size_t)s0 * X.d * (q_dtype == B2_F32 ? 4 : 2);  // bf16, fp16: 2
         if (X.n > 0) {
             dense_scores_kernel<<<grid_for(X.n * 32, 256, 148 * 8), 256, smem, stream>>>(X.store, X.dtype, X.n, X.d, qb, q_dtype,
                                                                                        sel, sc, metric, dense_ws);

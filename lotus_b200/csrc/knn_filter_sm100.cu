@@ -264,7 +264,8 @@ __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
     desc |= (uint64_t)2 << 61;                        // layout type: SWIZZLE_128B
     return desc;
 }
-// UMMA instruction descriptor: D fp32, A/B bf16 (1) or tf32 (2), both K-major, M = 128, N = 256.
+// UMMA instruction descriptor: D fp32, A/B bf16 (1) or tf32 (2), both K-major, M = 128, N = 256. fp16 operands (kind::f16,
+// format 0) use the bf16 descriptor with FilterParams::idesc_fmt_xor applied at run time (same instruction, same bytes).
 template <bool TF32, int M = BLOCK_M>
 __device__ __forceinline__ constexpr uint32_t make_idesc() {
     const uint32_t fmt = TF32 ? 2u : 1u;
@@ -303,7 +304,9 @@ struct FilterParams {
     int32_t* pair_j;
     unsigned long long* pair_count;   // total candidates found (may exceed pair_cap)
     unsigned long long pair_cap;
+    uint32_t idesc_fmt_xor;  // kind::f16 kernels: 0 for bf16 operands, F16_FMT_XOR for fp16 operands
 };
+constexpr uint32_t F16_FMT_XOR = (1u << 7) | (1u << 10);  // A/B format 1 (bf16) -> 0 (fp16)
 
 struct Ring {
     uint8_t* stage_base;
@@ -407,7 +410,8 @@ __device__ __forceinline__ void producer_loop(const CUtensorMap* tmap_q, const C
 // lane issues tcgen05.mma for every K-block, accumulating a 128x256 fp32 tile per CTA in TMEM.
 template <bool TF32, int NSTAGES, bool TWO>
 __device__ __forceinline__ void mma_loop(const FilterParams& p, const Ring& r, const Sched& sc) {
-    constexpr uint32_t idesc = make_idesc<TF32, TWO ? 2 * BLOCK_M : BLOCK_M>();
+    constexpr uint32_t idesc_c = make_idesc<TF32, TWO ? 2 * BLOCK_M : BLOCK_M>();
+    const uint32_t idesc = TF32 ? idesc_c : (idesc_c ^ p.idesc_fmt_xor);
     constexpr int SB = stage_bytes(TWO);
     const int n_items = num_items(p);
     int stage = 0;
@@ -953,10 +957,13 @@ PFN_encodeTiled get_encode_fn() {
 }
 
 // 2-D row-major matrix [rows, cols] with `pitch` elements per row; box = {128 bytes of K, box_rows rows}
-int make_tmap(CUtensorMap* map, const void* base, bool tf32, int64_t rows, int64_t cols, int64_t pitch, int box_rows) {
+int make_tmap(CUtensorMap* map, const void* base, int dtype, int64_t rows, int64_t cols, int64_t pitch, int box_rows) {
     PFN_encodeTiled enc = get_encode_fn();
     if (!enc) return B2_ECUDA;
-    const int esz = tf32 ? 4 : 2;
+    const int esz = dtype == B2_F32 ? 4 : 2;
+    const CUtensorMapDataType ttype = dtype == B2_F32   ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                      : dtype == B2_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                                        : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
     cuuint64_t gstride[1] = {(cuuint64_t)pitch * esz};
     cuuint32_t box[2] = {(cuuint32_t)(128 / esz), (cuuint32_t)box_rows};
@@ -965,7 +972,7 @@ int make_tmap(CUtensorMap* map, const void* base, bool tf32, int64_t rows, int64
         set_error("TMA operand not 16-byte aligned (base %p, pitch %lld B)", base, (long long)gstride[0]);
         return B2_EINVAL;
     }
-    CUresult r = enc(map, tf32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
+    CUresult r = enc(map, ttype, 2,
                      const_cast<void*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
@@ -1151,10 +1158,11 @@ int launch_knn_filter(const MatView& X, const void* q_filt, int64_t q_pitch, int
     const int kb_elems = tf32 ? 32 : 64;
     CUtensorMap tq, tx;
     const int64_t op_cols = X.d;
-    B2_TRY(make_tmap(&tq, q_filt, tf32, nq, op_cols, q_pitch, BLOCK_M));
+    B2_TRY(make_tmap(&tq, q_filt, X.filt_dtype, nq, op_cols, q_pitch, BLOCK_M));
     // pair mode: each CTA of the pair loads HALF of the 256-row corpus tile
-    B2_TRY(make_tmap(&tx, X.filt, tf32, X.n, op_cols, X.filt_pitch, two_cta ? BLOCK_N / 2 : BLOCK_N));
+    B2_TRY(make_tmap(&tx, X.filt, X.filt_dtype, X.n, op_cols, X.filt_pitch, two_cta ? BLOCK_N / 2 : BLOCK_N));
     FilterParams p;
+    p.idesc_fmt_xor = X.filt_dtype == B2_F16 ? F16_FMT_XOR : 0u;
     p.xnorm = X.norm2;
     p.cand_score = cand_score;
     p.cand_id = cand_id;
@@ -1252,16 +1260,17 @@ int launch_pair_filter(const MatView& X, float thr, int part, int nparts, int32_
     const bool tf32 = X.filt_dtype == B2_F32;
     const int kb_elems = tf32 ? 32 : 64;
     CUtensorMap tq, tx;
-    B2_TRY(make_tmap(&tq, X.filt, tf32, X.n, X.d, X.filt_pitch, BLOCK_M));
-    B2_TRY(make_tmap(&tx, X.filt, tf32, X.n, X.d, X.filt_pitch, BLOCK_N));
+    B2_TRY(make_tmap(&tq, X.filt, X.filt_dtype, X.n, X.d, X.filt_pitch, BLOCK_M));
+    B2_TRY(make_tmap(&tx, X.filt, X.filt_dtype, X.n, X.d, X.filt_pitch, BLOCK_N));
     FilterParams p;
     memset(&p, 0, sizeof(p));
+    p.idesc_fmt_xor = X.filt_dtype == B2_F16 ? F16_FMT_XOR : 0u;
     p.nq = (int32_t)X.n;
     p.n = (int32_t)X.n;
     p.num_kb = (int32_t)ceil_div(X.d, kb_elems);
     static const bool two = [] { const char* e = getenv("B2_PAIR_2CTA"); return e ? atoi(e) != 0 : true; }();  // default: CTA pairs
     const bool two_cta = two && ceil_div(X.n, BLOCK_M) >= 2;
-    if (two_cta) B2_TRY(make_tmap(&tx, X.filt, tf32, X.n, X.d, X.filt_pitch, BLOCK_N / 2));  // each CTA stages half a corpus tile
+    if (two_cta) B2_TRY(make_tmap(&tx, X.filt, X.filt_dtype, X.n, X.d, X.filt_pitch, BLOCK_N / 2));  // each CTA stages half a corpus tile
     p.n_mtiles = (int32_t)ceil_div(X.n, BLOCK_M);
     p.n_munits = two_cta ? (p.n_mtiles + 1) / 2 : p.n_mtiles;
     p.n_ntiles = (int32_t)ceil_div(X.n, BLOCK_N);

@@ -23,8 +23,14 @@ def shard_bounds(n: int, world: int, rank: int) -> tuple[int, int]:
     return lo, lo + base + (1 if rank < rem else 0)
 
 
+def _torch_code(dtype):
+    """Native element-type code of a torch dtype (None for the ones the library does not take)."""
+    import torch
+    return {torch.float32: nv.F32, torch.bfloat16: nv.BF16, torch.float16: nv.F16}.get(dtype)
+
+
 class ShardedIndex:
-    """Each rank holds `local_rows` (a torch CUDA tensor [n_local, d], bf16 or fp32) = its slice of the corpus."""
+    """Each rank holds `local_rows` (a torch CUDA tensor [n_local, d], fp32, bf16 or fp16) = its slice of the corpus."""
 
     def __init__(self, local_rows, row_offset: int, metric: int = nv.METRIC_IP, group=None):
         import torch
@@ -36,9 +42,9 @@ class ShardedIndex:
         self.rank = dist.get_rank(group) if self.world > 1 else 0
         assert local_rows.is_cuda and local_rows.dim() == 2 and local_rows.is_contiguous()
         self.device = local_rows.device.index if local_rows.device.index is not None else torch.cuda.current_device()
-        self.dtype = nv.BF16 if local_rows.dtype == torch.bfloat16 else nv.F32
-        if self.dtype == nv.F32 and local_rows.dtype != torch.float32:
-            raise TypeError("corpus must be float32 or bfloat16")
+        self.dtype = _torch_code(local_rows.dtype)
+        if self.dtype is None:
+            raise TypeError("corpus must be float32, bfloat16 or float16")
         self.metric = metric
         self.row_offset = int(row_offset)
         n, d = local_rows.shape
@@ -54,14 +60,16 @@ class ShardedIndex:
             self.shard_offsets[0] = self.row_offset
 
     def search(self, q, k: int, ids=None):
-        """q: torch CUDA tensor [nq, d] (bf16 or fp32), replicated on every rank.
+        """q: torch CUDA tensor [nq, d] (fp32, bf16 or fp16), replicated on every rank.
         ids: optional GLOBAL row ids (ascending, replicated): each rank keeps those inside its row range — the sharded
         form of FaissVS.__call__(ids=...) (faiss_vs.py:57-72).
         -> (scores [nq,k] float32, idx [nq,k] int64) CUDA tensors holding the GLOBAL top-k on every rank."""
         torch = self.torch
         assert q.is_cuda and q.is_contiguous() and q.shape[1] == self.d
         nq = q.shape[0]
-        q_dtype = nv.BF16 if q.dtype == torch.bfloat16 else nv.F32
+        q_dtype = _torch_code(q.dtype)
+        if q_dtype is None:
+            raise TypeError("queries must be float32, bfloat16 or float16")
         stream = torch.cuda.current_stream().cuda_stream
         if ids is None and self.world > 1:
             return self._search_packed(q, k)
@@ -97,7 +105,7 @@ class ShardedIndex:
         """The whole-index step: local search -> ONE all-gather of 8-byte (score, local id) entries -> single-kernel k-way merge."""
         torch = self.torch
         nq = q.shape[0]
-        q_dtype = nv.BF16 if q.dtype == torch.bfloat16 else nv.F32
+        q_dtype = _torch_code(q.dtype)
         stream = torch.cuda.current_stream().cuda_stream
         timing = os.environ.get("B2_SHARD_TIMING") == "1"
         if timing:
@@ -248,7 +256,7 @@ def sharded_kmeans(index: "nv.Index", n_total: int, row_offset: int, k: int, nit
     cent_h = np.zeros((k, d), dtype=np.float32)
     if mine.any():
         rows = index.gather(want[mine] - row_offset)
-        cent_h[mine] = nv.bf16_bits_to_f32(rows) if index.dtype == nv.BF16 else rows
+        cent_h[mine] = nv.bits_to_f32(rows, index.dtype)
     cent = torch.from_numpy(cent_h).to(dev)
     if world > 1:
         dist.all_reduce(cent, group=group)  # each row is non-zero on exactly one rank

@@ -40,13 +40,18 @@ class SemDedupByDataframe:
         if n == 0:
             return self._obj
         rows = np.asarray(self._obj.index, dtype=np.int64)  # positions into the index (un-reset RangeIndex contract)
+        pairs = None
         if hasattr(vs, "threshold_pairs"):
             try:
-                pi, pj = vs.threshold_pairs(float(threshold))   # pairs over INDEX positions, i < j
+                pairs = vs.threshold_pairs(float(threshold))   # pairs over INDEX positions, i < j
+            except NotImplementedError:
+                pairs = None  # e.g. an SQfp16 store, whose relation is asymmetric: the reference relation below
             except nv.NativeError as e:
                 if e.code in (nv.EINVAL, nv.ERANGE):  # e.g. an L2 index: the relation is defined on inner products
                     raise ValueError(e.msg) from e
                 raise
+        if pairs is not None:
+            pi, pj = pairs
             # restrict to this frame's rows and translate to frame-local row numbers
             pos = np.full(int(max(rows.max(), pi.max() if len(pi) else 0, pj.max() if len(pj) else 0)) + 1, -1, dtype=np.int64)
             pos[rows] = np.arange(n)
@@ -54,7 +59,7 @@ class SemDedupByDataframe:
             ok = (li >= 0) & (lj >= 0)
             li, lj = li[ok], lj[ok]
         else:
-            # any other VS (e.g. the reference's FaissVS): the reference's own relation — every row against every row of the
+            # any other VS (e.g. the reference's FaissVS), or a store without a symmetric all-pairs relation: the reference's own relation — every row against every row of the
             # frame through vs(..., K=n, ids=rows) (sem_dedup.py:45 via sem_sim_join.py:132-134), `_scores > threshold` (:46)
             qv = vs.get_vectors_from_index(col_index_dir, rows.tolist())
             out = vs(qv, n, ids=rows.tolist())

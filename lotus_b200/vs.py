@@ -77,15 +77,21 @@ class BF16Backed(np.ndarray):
         return np.ascontiguousarray(f32, dtype=np.float32).view(BF16Backed)
 
 
-def _to_host_matrix(a: Any, want_bf16: bool, exact_bf16_ok: bool = False, scratch: "dict | None" = None):
+def _to_host_matrix(a: Any, want_bf16: bool, exact_bf16_ok: bool = False, scratch: "dict | None" = None, want_f16: bool = False,
+                    exact_f16_ok: bool = False):
     """-> (array for the C-ABI, native dtype code, float32 view of the stored values).
     exact_bf16_ok: when every float32 value is bfloat16-representable (e.g. vectors fetched from a bf16 index,
     sem_sim_join.py:112-118 -> :130-134) ship the exact 2-byte patterns instead: half the H2D bytes and the exact-operand
-    error bound in the certificate. Decided from the values themselves on every call (one threaded host pass)."""
+    error bound in the certificate. Decided from the values themselves on every call (one threaded host pass).
+    want_f16 / exact_f16_ok: the same for fp16 (IEEE binary16, rounded to nearest even by numpy); want_f16 rounds, and a value
+    beyond fp16's finite range raises ValueError."""
     try:
         import torch
         if isinstance(a, torch.Tensor):
             t = a.detach()
+            if t.dtype == torch.float16 and (want_f16 or exact_f16_ok):
+                bits = t.contiguous().cpu().view(torch.int16).numpy().view(np.uint16)
+                return bits, nv.F16, nv.f16_bits_to_f32(bits)
             if t.dtype == torch.bfloat16 or want_bf16:
                 bits = t.to(torch.bfloat16).contiguous().cpu().view(torch.int16).numpy().view(np.uint16)
                 return bits, nv.BF16, nv.bf16_bits_to_f32(bits)
@@ -95,6 +101,14 @@ def _to_host_matrix(a: Any, want_bf16: bool, exact_bf16_ok: bool = False, scratc
     f = np.ascontiguousarray(np.asarray(a), dtype=np.float32)  # faiss casts whatever it is given to float32
     if f.ndim != 2:
         raise ValueError(f"embeddings must be 2-D, got shape {f.shape}")
+    if want_f16:
+        bits = nv.f32_to_f16_bits(f)
+        _check_f16_range(bits)
+        return bits, nv.F16, nv.f16_bits_to_f32(bits)
+    if exact_f16_ok and f.size:
+        bits = nv.f32_to_f16_bits(f)
+        if np.array_equal(nv.f16_bits_to_f32(bits), f):
+            return bits, nv.F16, f
     if want_bf16:
         bits = nv.f32_to_bf16_bits(f)
         return bits, nv.BF16, nv.bf16_bits_to_f32(bits)
@@ -109,6 +123,13 @@ def _to_host_matrix(a: Any, want_bf16: bool, exact_bf16_ok: bool = False, scratc
         if exact:
             return bits, nv.BF16, f
     return f, nv.F32, f
+
+
+def _check_f16_range(bits: np.ndarray) -> None:
+    """An fp16 store holds finite values only: faiss's SQfp16 would store inf for |x| >= 65520; this store refuses."""
+    if bits.size and ((bits & 0x7C00) == 0x7C00).any():
+        raise ValueError("embeddings have values beyond the finite range of fp16 (|x| >= 65520, or inf / NaN); an fp16 store "
+                         "(dtype='f16' or factory_string='SQfp16') cannot hold them")
 
 
 class MultiDeviceIndex:
@@ -152,7 +173,7 @@ class MultiDeviceIndex:
         ids = np.asarray(ids, dtype=np.int64)
         if len(ids) and (ids.min() < 0 or ids.max() >= self.n):
             raise nv.NativeError(nv.ERANGE, f"ids contains a position outside [0, {self.n})")
-        out = np.empty((len(ids), self.d), dtype=np.float32 if self.dtype == nv.F32 else np.uint16)
+        out = np.empty((len(ids), self.d), dtype=np.float32 if self.dtype == nv.F32 else np.uint16)  # BF16 / F16: bit patterns
         for g, (lo, hi) in enumerate(self.bounds):
             m = (ids >= lo) & (ids < hi)
             if m.any():
@@ -195,8 +216,10 @@ class B200VS(VS):
     """Flat (brute-force, exact) vector store on one B200 (or, with devices=[...], row-sharded over several from one process).
 
     Args mirror FaissVS(factory_string="Flat", metric=faiss.METRIC_INNER_PRODUCT) (faiss_vs.py:14).
-    dtype: "f32" (store what faiss would: float32), "bf16" (round the corpus to bfloat16 once; exact search
-    over those values), or "auto" (bf16 only when handed a bf16 tensor).
+    factory_string: "Flat", or "SQfp16" — faiss IndexScalarQuantizer(d, QT_fp16): the rows are stored rounded to fp16, fp32
+    queries are scored exactly against them, and `get_vectors_from_index` returns the ORIGINAL embeddings (faiss_vs.py:38-41).
+    dtype: "f32" (store what faiss would: float32), "bf16" / "f16" (round the corpus to bfloat16 / fp16 once; exact search
+    over those values), or "auto" (bf16 only when handed a bf16 tensor). "SQfp16" implies "f16".
     """
 
     accepts_id_arrays = True  # `ids=` may be a numpy int64 array (the operators then skip building a Python list)
@@ -204,12 +227,17 @@ class B200VS(VS):
     def __init__(self, factory_string: str = "Flat", metric: int = METRIC_INNER_PRODUCT, dtype: str = "auto",
                  device: int = 0, cache_size: int = 4, devices: "list[int] | None" = None):
         super().__init__()
-        if factory_string != "Flat":
-            raise ValueError(f"B200VS implements the flat (exact) index only; factory_string={factory_string!r}")
+        if factory_string not in (faiss_io.FLAT, faiss_io.SQFP16):
+            raise ValueError(f"B200VS implements the flat (exact) index types 'Flat' and 'SQfp16' only; factory_string={factory_string!r}")
         if metric not in (METRIC_INNER_PRODUCT, METRIC_L2):
             raise ValueError("metric must be METRIC_INNER_PRODUCT (0) or METRIC_L2 (1)")
-        if dtype not in ("auto", "f32", "bf16"):
-            raise ValueError("dtype must be 'auto', 'f32' or 'bf16'")
+        if dtype not in ("auto", "f32", "bf16", "f16"):
+            raise ValueError("dtype must be 'auto', 'f32', 'bf16' or 'f16'")
+        self.sq = factory_string == faiss_io.SQFP16
+        if self.sq:
+            if dtype not in ("auto", "f16"):
+                raise ValueError(f"factory_string='SQfp16' stores fp16 rows; dtype={dtype!r} contradicts it")
+            dtype = "f16"
         self.factory_string = factory_string
         self.metric = metric
         self.dtype = dtype
@@ -226,21 +254,25 @@ class B200VS(VS):
     def _build(self, embeddings: Any) -> nv.Index:
         nv.require_device()
         t = _cuda_tensor(embeddings)
+        f16 = self.dtype == "f16"
         if self.devices and len(self.devices) > 1:
             want16 = self.dtype == "bf16"
             if t is not None:
                 import torch
                 want16 = want16 or (self.dtype == "auto" and t.dtype == torch.bfloat16)
-            host, code, _ = _to_host_matrix(embeddings, want16)
+            host, code, _ = _to_host_matrix(embeddings, want16, want_f16=f16)
             return MultiDeviceIndex(host, code, self.metric, self.devices)  # type: ignore[return-value]
         if t is not None and t.dim() == 2 and t.device.index == self.device:
             # device hand-off: the encoder's output never visits the host on its way into the index
             import torch
             want = torch.bfloat16 if (self.dtype == "bf16" or (self.dtype == "auto" and t.dtype == torch.bfloat16)) else torch.float32
+            want = torch.float16 if f16 else want
             t = t.detach().to(want).contiguous()
-            return nv.Index(None, nv.BF16 if want == torch.bfloat16 else nv.F32, self.metric, self.device,
-                            on_device_ptr=t.data_ptr(), n=t.shape[0], d=t.shape[1])
-        host, code, _ = _to_host_matrix(embeddings, self.dtype == "bf16")
+            if f16 and t.numel() and not bool(torch.isfinite(t).all()):
+                _check_f16_range(np.array([0x7C00], dtype=np.uint16))  # raises the range error
+            code = {torch.bfloat16: nv.BF16, torch.float16: nv.F16}.get(want, nv.F32)
+            return nv.Index(None, code, self.metric, self.device, on_device_ptr=t.data_ptr(), n=t.shape[0], d=t.shape[1])
+        host, code, _ = _to_host_matrix(embeddings, self.dtype == "bf16", want_f16=f16)
         return nv.Index(host, code, self.metric, self.device)
 
     def _remember(self, index_dir: str, idx: nv.Index, vecs: Any) -> None:
@@ -262,7 +294,7 @@ class B200VS(VS):
         """faiss_vs.py:22-30: build the flat index, persist `vecs` (pickle) and `index` (faiss IndexFlat file)."""
         idx = self._build(embeddings)
         _, _, f32 = _to_host_matrix(embeddings, False)
-        faiss_io.write_index_dir(index_dir, embeddings, f32, self.metric)
+        faiss_io.write_index_dir(index_dir, embeddings, f32, self.metric, kind=self.factory_string)
         self.b2_index = idx
         self.vecs = embeddings
         self.index_dir = index_dir
@@ -282,10 +314,12 @@ class B200VS(VS):
                 self._cache.move_to_end(key)
                 self.index_dir, self.b2_index, self.vecs = index_dir, hit[1], hit[2]
                 return
-        vecs, x, metric = faiss_io.read_index_dir(index_dir)
+        vecs, x, metric, kind = faiss_io.read_index_dir(index_dir, with_kind=True)
         if metric != self.metric:
             raise ValueError(f"index at {index_dir} was built with metric {metric}, this store uses {self.metric}")
-        idx = self._build(vecs if self.dtype != "f32" else x)
+        if kind != self.factory_string:
+            raise ValueError(f"index at {index_dir} is a {kind!r} index, this store uses factory_string={self.factory_string!r}")
+        idx = self._build(x if (self.sq or self.dtype == "f32") else vecs)
         self.index_dir, self.b2_index, self.vecs = index_dir, idx, vecs
         self._remember(index_dir, idx, vecs)
 
@@ -310,8 +344,22 @@ class B200VS(VS):
         not change which index is loaded."""
         idx = self._entry_for(index_dir)
         ids_a = np.asarray(list(ids) if not isinstance(ids, np.ndarray) else ids, dtype=np.int64)
+        if self.sq:  # SQfp16: the pickle keeps the original embeddings and the reference returns those, not the fp16 rows
+            orig = self._originals(index_dir)
+            if len(ids_a) and (ids_a.min() < -len(orig) or ids_a.max() >= len(orig)):
+                raise IndexError(f"ids contains a position outside [0, {len(orig)})")
+            return orig[ids_a]
         out = idx.gather(ids_a)
+        if idx.dtype == nv.F16:
+            return nv.f16_bits_to_f32(out)
         return BF16Backed.wrap(nv.bf16_bits_to_f32(out)) if idx.dtype == nv.BF16 else out
+
+    def _originals(self, index_dir: str) -> np.ndarray:
+        """The `vecs` of `index_dir` (what index() was given) as float32 — faiss casts whatever it is given to float32."""
+        key = os.path.abspath(index_dir)
+        hit = self._cache.get(key)
+        vecs = hit[2] if hit is not None else self.vecs
+        return _to_host_matrix(vecs, False)[2]
 
     def __call__(self, query_vectors: Any, K: int, ids: list[int] | None = None, **kwargs: Any) -> RMOutput:
         """faiss_vs.py:43-77. Returns float32 distances [Q,K] and int64 indices [Q,K] (global ids; -1 = no result).
@@ -322,7 +370,8 @@ class B200VS(VS):
         t = _cuda_tensor(query_vectors)
         if t is not None and ids_a is None and t.dim() == 2 and t.device.index == self.device and not isinstance(self.b2_index, MultiDeviceIndex):
             return self._call_device(t, int(K))
-        q, code, _ = _to_host_matrix(query_vectors, False, exact_bf16_ok=self.b2_index.dtype == nv.BF16, scratch=self._scratch)
+        q, code, _ = _to_host_matrix(query_vectors, False, exact_bf16_ok=self.b2_index.dtype == nv.BF16, scratch=self._scratch,
+                                     exact_f16_ok=self.b2_index.dtype == nv.F16)
         if q.shape[1] != self.b2_index.d:
             raise ValueError(f"query dimension {q.shape[1]} does not match the index dimension {self.b2_index.d}")
         try:
@@ -340,8 +389,10 @@ class B200VS(VS):
         if t.shape[1] != self.b2_index.d:
             raise ValueError(f"query dimension {t.shape[1]} does not match the index dimension {self.b2_index.d}")
         q = t.detach()
-        q = q.contiguous() if q.dtype in (torch.float32, torch.bfloat16) else q.to(torch.float32).contiguous()
-        code = nv.BF16 if q.dtype == torch.bfloat16 else nv.F32
+        # fp16 queries stream in place against an fp16 store; any other store sees them widened to fp32, as before
+        native = (torch.float32, torch.bfloat16, torch.float16) if self.b2_index.dtype == nv.F16 else (torch.float32, torch.bfloat16)
+        q = q.contiguous() if q.dtype in native else q.to(torch.float32).contiguous()
+        code = {torch.bfloat16: nv.BF16, torch.float16: nv.F16}.get(q.dtype, nv.F32)
         out_s = torch.empty((q.shape[0], K), dtype=torch.float32, device=q.device)
         out_i = torch.empty((q.shape[0], K), dtype=torch.int64, device=q.device)
         try:
@@ -355,6 +406,10 @@ class B200VS(VS):
 
     # -- extensions used by the re-registered operators --------------------------------------------------------------
     def threshold_pairs(self, threshold: float):
+        if self.sq:
+            # the reference relation x_i . fp16(x_j) > t is asymmetric (fp32 query against the fp16 row); the all-pairs kernel is
+            # symmetric. sem_dedup then runs the reference's own relation through __call__ (O(n^2), like the reference).
+            raise NotImplementedError("threshold_pairs is not available on an SQfp16 store (asymmetric relation)")
         if self.b2_index is None:
             raise ValueError("Index not loaded")
         return self.b2_index.threshold_pairs(threshold)
@@ -362,7 +417,17 @@ class B200VS(VS):
     def kmeans(self, ids: Any, ncentroids: int, niter: int = 20, seed: int = 1234, full_lloyd: bool = False):
         if self.b2_index is None:
             raise ValueError("Index not loaded")
-        return self.b2_index.kmeans(ncentroids, niter=niter, seed=seed, ids=np.asarray(ids, dtype=np.int64), full_lloyd=full_lloyd)
+        ids_a = np.asarray(ids, dtype=np.int64)
+        if self.sq:
+            # lotus.utils.cluster trains faiss.Kmeans on get_vectors_from_index, i.e. on the original embeddings: a temporary
+            # fp32 index over vecs[ids], not the fp16 rows
+            assert self.index_dir is not None
+            tmp = nv.Index(np.ascontiguousarray(self._originals(self.index_dir)[ids_a]), nv.F32, self.metric, self.device)
+            try:
+                return tmp.kmeans(ncentroids, niter=niter, seed=seed, full_lloyd=full_lloyd)
+            finally:
+                tmp.close()
+        return self.b2_index.kmeans(ncentroids, niter=niter, seed=seed, ids=ids_a, full_lloyd=full_lloyd)
 
     def close(self) -> None:
         for _, idx, _ in self._cache.values():
